@@ -3,6 +3,7 @@
     python bench.py                                                  # BASELINE configs[1]: 1 deg, 102->78, batch 8, default path
     python bench.py --grid 0.25deg --batch 4 --precision bf16        # BASELINE configs[2]
     python bench.py --impl reference --steps 2 --warmup 1            # the reference's CPU forward on the host cores
+    python bench.py --dump-outputs DIR                               # also writes the last timed step's forecast to DIR
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N [--grid 0.25deg --batch 4 --precision bf16]
 
 The model is built exactly as a user of the reference builds it -- `GraphWeatherForecaster(lat_lons)`, no extra keyword --
@@ -56,6 +57,21 @@ def grid_quarter_deg():
 
 
 GRIDS = {"1deg": grid_1deg, "0.25deg": grid_quarter_deg}
+DUMP_BYTES = 48 * 2**20  # --dump-outputs writes at most this much data (under 64 MB with the .npy headers)
+
+
+def output_sample(y):
+    """Host copy of what one step returned, for --dump-outputs.  A forecast [B, N, F] is kept whole when it fits DUMP_BYTES,
+    else at a fixed sorted sample of grid points (PCG64 seed 0, the same points for every sample); a loss is kept as is."""
+    y = y.detach()
+    if y.dim() != 3:
+        return {"loss": y.double().cpu().numpy()}
+    b, n, f = y.shape
+    k = min(n, DUMP_BYTES // (b * f * 4))
+    if k < n:
+        idx = np.sort(np.random.Generator(np.random.PCG64(0)).choice(n, k, replace=False))
+        y = y[:, torch.from_numpy(idx).to(y.device)]
+    return {"forecast": y.float().cpu().numpy()}
 
 
 def algorithmic_flops(n, ed):
@@ -242,7 +258,13 @@ def main():
                     help="transport of the gather boundary: fused into the forecast's last kernel (NVLink multicast / peer stores), copy engines, or NCCL")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-check", action="store_true", help="skip the oracle comparison of this run's output")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (float32 forecast, "
+                    "sampled at fixed grid points above 48 MiB; float64 loss with --boundary loss) to compare two builds")  # fmt: skip
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if a.batch is None:
         a.batch = 8 if a.grid == "1deg" else 4
     if a.precision is None:
@@ -390,7 +412,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         cur = torch.cuda.current_stream(dev)
         if gather is not None:
             gather.wait()  # the timed region ends when the last gather has landed ...
@@ -401,7 +423,7 @@ def main():
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)  # max over ranks
         sync_all()
-        return float(ms.item())
+        return float(ms.item()), out
 
     warm = max(3, a.warmup)
     for _ in range(warm):
@@ -410,14 +432,16 @@ def main():
     plan.timing_enable(True)
     _capi.launch_count_reset()
     with ClockSampler(local) as clk:
-        ms_total = timed(step_resident, a.steps)
+        ms_total, y_last = timed(step_resident, a.steps)
+    # copied now: the end-to-end steps below reuse the gather buffers
+    dump = output_sample(y_last) if (a.dump_outputs and rank == 0) else None
     launches = _capi.launch_count()
     tags = plan.timing_read()
     plan.timing_enable(False)
     plan.status()  # raises if any kernel flagged fp16-range overflow or a pipeline fault
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, a.steps)
+    ms_e2e, _ = timed(step_e2e, a.steps)
     ms_step = ms_total / a.steps
     value = world * a.steps / (ms_total / 1000.0)
     e2e_value = world * a.steps / (ms_e2e / 1000.0)
@@ -495,6 +519,10 @@ def main():
         line["cpu_baseline"] = {"value": r["steps_per_s"], "unit": "steps/s", "cores": r["cores"], "kind": r["kind"], "seconds_per_forward": r["seconds_per_forward"],
                                 "sample": f"reference forward on {sample_b} of the {a.batch} samples per timed forward ({r['warmup']} warm-up + {r['steps']} timed); steps/s = samples/s / {a.batch}; "
                                           "`bench.py --impl reference` times the full batch"}  # fmt: skip
+    if dump is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     emit(line)
     if world > 1:
         dist.destroy_process_group()

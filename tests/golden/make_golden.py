@@ -8,6 +8,7 @@ Each fixture stores the config, the seed and the reference outputs (plus sub-sam
 inputs are regenerated from the seed by oracle/weights.py when the fixture is checked.
 """
 
+import hashlib
 import json
 import os
 import sys
@@ -176,6 +177,23 @@ def run_constraints(R, name="forecaster_constraints_10deg_b2"):
         hr=hr.numpy(), lr=lr.numpy(), **layer_out)  # fmt: skip
 
 
+def run_init(R, name="forecaster_init_seed42"):
+    """GraphWeatherForecaster's default initialisation under torch.manual_seed(42) on a 30-degree grid.  The full state_dict is
+    ~31 MB, so the fixture keeps the key order, the shapes, 16 seeded values and the sha256 of the fp32 bytes of every tensor."""
+    seed, step, per = 42, 30, 16
+    torch.manual_seed(seed)
+    sd = R.GraphWeatherForecaster(grid(step)).state_dict()
+    rng = np.random.Generator(np.random.PCG64(0))
+    vals = [v.detach().contiguous().numpy() for v in sd.values()]
+    assert all(v.dtype == np.float32 for v in vals)
+    index = np.stack([rng.integers(0, v.size, per) for v in vals])
+    np.savez_compressed(
+        os.path.join(HERE, name + ".npz"), config=json.dumps(dict(seed=seed, step=step, keys=list(sd.keys()), shapes=[list(v.shape) for v in vals])),
+        sample_index=index, sample=np.stack([v.reshape(-1)[i] for v, i in zip(vals, index)]),
+        sha256=np.array([hashlib.sha256(v.tobytes()).hexdigest() for v in vals]))  # fmt: skip
+    print(name, len(vals), "tensors", sum(v.size for v in vals), "values")
+
+
 def regional_region():
     """A 0.5-degree box over western Europe plus a few scattered points (one near a pentagon): the movable domain of the test."""
     ll = [(38.0 + 0.5 * i, -12.0 + 0.5 * j) for i in range(40) for j in range(61)]
@@ -224,3 +242,5 @@ if __name__ == "__main__":
         run_constraints(R)
     if not only or "regional" in only:
         run_regional(R)
+    if not only or "init" in only:
+        run_init(R)
